@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — global-BA LM iterations / second on synthetic BA problems of the BASELINE.json shapes.
 
-    python bench.py --gpus N --steps K --warmup W [--workload cfg5] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload cfg5] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one Global-BA solve: optimizer.optimize(20) of Optimizer::MapFusionGBA (S/Optimizer.cpp:797) on the
 workload (default cfg5 = synthetic 10k keyframes x 1M landmarks x 20M observations, the only BASELINE config defined
@@ -16,10 +16,14 @@ compares with the CPU oracle ("parity" in the JSON line; a failure exits 3 after
 "cfg4" (the >= 50x target shape: resident, end to end, full-size CPU) and "frontend" (ms per frame / call of the ORB extractor and
 the BoW matchers next to the CPU oracle).
 
+--dump-outputs DIR writes what the last timed step computed, as a caller of ccm_ba_optimize receives it, to DIR/<name>.npy (rank 0;
+the state is downloaded after the step's closing event, so the timed figure does not include it).  The workloads are seeded, so two
+builds run with the same arguments can be compared output for output.
+
 --impl reference times the reference's CPU algorithm (the dependency-free oracle port, bit-identical to the reference's own
 Optimizer.cpp + g2o compiled over a stand-in Eigen and twice as fast as that build; the reference proper cannot be built here:
 no Eigen) on the host, single thread — the reference build is single-threaded by construction (cslam/thirdparty/g2o/config.h:4)
-— on the FULL workload with the same stop rule (about 100 s per Global BA of cfg5).
+— on the FULL workload with the same stop rule (about 100 s per Global BA of cfg5, so --steps should stay small there).
 """
 from __future__ import annotations
 
@@ -118,13 +122,13 @@ def run_reference(args, rank, world):
     """Reference arm: the reference's CPU algorithm (oracle port, direct sparse LDL^T like g2o's LinearSolverEigen) on the FULL
     workload with the same stop rule as our arm (optimize(20): cfg5 ends after 8 LM iterations by the three-strike rule), timed
     around the optimize() equivalent exactly as the reference times it (S/Optimizer.cpp:796-801).  One Global BA of cfg5 is about
-    100 s of single-thread CPU work, so at most CCM_REF_STEPS (default 2) steps are timed whatever --steps asks for."""
+    100 s of single-thread CPU work."""
     if rank != 0:
         return
     from oracle import pyoracle
     p = synth.make_config(args.workload)
     delta = float(np.float32(np.sqrt(5.99)))
-    steps = max(1, min(args.steps, int(os.environ.get("CCM_REF_STEPS", "2"))))
+    steps = args.steps
     small = synth.make_config("small")
     for _ in range(min(args.warmup, 1)):
         pyoracle.ba_solve(small, iterations=2, huber_delta=delta)   # page in the library; the CPU arm has no caches to warm
@@ -249,6 +253,29 @@ def cfg4_block(api):
                        "max_rel_pose": float(np.abs(Tg - To).max() / max(1.0, np.abs(To).max()))}}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, r):
+    """The arrays ccm_ba_optimize hands back (poses, points, LM trace) and its counters, as float64 .npy files.  An array that would take
+    the total past DUMP_LIMIT_BYTES is cut to a seeded sample of its rows, and the row indices go to <name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"poses": r["poses"], "points": r["points"], "trace": r["trace"],
+              "summary": np.array([r["iters_done"], r["trials_total"], r["pcg_iters_total"], r["pcg_not_converged"],
+                                   r["chi2_initial"], r["chi2_final"], r["lambda_final"]])}
+    budget = DUMP_LIMIT_BYTES
+    for name in ("summary", "trace", "poses", "points"):
+        a = np.ascontiguousarray(arrays[name], np.float64)
+        if a.nbytes > budget:
+            keep = budget // (a.nbytes // len(a) + 8)
+            rows = np.sort(np.random.default_rng(0).choice(len(a), size=keep, replace=False)).astype(np.int64)
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows)
+            budget -= rows.nbytes
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        budget -= a.nbytes
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -260,7 +287,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the pre-flight parity block (oracle on rank 0, about 10 s)")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg4 and front-end sub-blocks of the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -309,11 +339,11 @@ def main():
     info = h.info()
     small = info["device_bytes"] < (200 << 20)  # inputs not larger than L2 -> flush between iterations
 
-    def one_step():
+    def one_step(want_state=False):
         h.reset()
         if small:
             api.l2_flush()
-        return h.optimize(iterations=LM_ITERS, huber_delta=delta, want_state=False)
+        return h.optimize(iterations=LM_ITERS, huber_delta=delta, want_state=want_state)
 
     for _ in range(max(args.warmup, 3)):
         one_step()
@@ -323,9 +353,9 @@ def main():
     launches0 = api.kernel_launches()
     t_dev_ms, it_tot, tr_tot, pcg_tot, pcg_nc = 0.0, 0, 0, 0, 0
     wall0 = time.perf_counter()
-    for _ in range(args.steps):
+    for step in range(args.steps):
         barrier()
-        r = one_step()
+        r = one_step(want_state=bool(args.dump_outputs) and step == args.steps - 1)
         t_dev_ms += max_over_ranks(r["t_optimize_event_ms"])  # CUDA events on the launching stream, max over ranks
         if rank == 0:
             print("[bench] step: device %.1f ms (host wall of the call %.1f ms), %d LM iterations, %d PCG iterations" % (
@@ -338,6 +368,8 @@ def main():
     h.set_profile(False)
     clocks = sampler.stop() if sampler else None
     value = it_tot / (t_dev_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r)
 
     # ---- end-to-end through the one-shot C ABI call with host buffers (pinned), copies inside the timed region
     arrs = [p.poses, p.intr, p.fixed, p.points, p.obs_kf, p.obs_mp, p.obs_uv, p.obs_w]

@@ -735,6 +735,12 @@ def _plain(desc, angle, octave=None, xy=None):
                 angle=angle)
 
 
+def ref_descriptor_distance(a, b):
+    """ORBmatcher::DescriptorDistance of the matcher library"""
+    a = np.ascontiguousarray(a, np.uint8); b = np.ascontiguousarray(b, np.uint8)
+    return ref_match().ref_descriptor_distance(_p(a), _p(b))
+
+
 def ref_match_bow_kf_frame(desc_kf, has_mp, ang_kf, fv_kf, desc_f, ang_f, fv_f, nnratio=0.7, check_ori=True):
     keep = []; K = ref_image_struct(_plain(desc_kf, ang_kf), keep, fv=fv_kf); F = ref_image_struct(_plain(desc_f, ang_f), keep, fv=fv_f)
     has = np.ascontiguousarray(has_mp, np.uint8); out = np.empty(len(desc_f), np.int32)

@@ -2,7 +2,7 @@
 cslam/thirdparty/DBoW2 compiled where it lies (oracle/Makefile `ref`, stand-in OpenCV header oracle/ref_stub/) — the one piece of the
 hot path's neighbourhood that builds in this image.  Vocabulary text loader, word / node numbering, tree descent with its first-minimum
 rule, FORB::distance, BowVector / FeatureVector arithmetic for every scoring and weighting type: exact, doubles bit for bit.
-Skipped where neither /root/reference nor a prebuilt library is present."""
+The reference's outputs are stored under tests/golden/reference (tests/reference_outputs.py)."""
 import os
 import tempfile
 
@@ -10,13 +10,12 @@ import numpy as np
 import pytest
 
 from ccm_slam_b200 import synth_match as sm
+from tests.reference_outputs import Recorded, same
 
 
 @pytest.fixture(scope="module")
 def ref(oracle):
-    if oracle.ref_dbow2() is None:
-        pytest.skip("reference DBoW2 library not available (no /root/reference, no prebuilt oracle/_ref)")
-    return oracle
+    return Recorded(oracle, __file__, oracle.ref_dbow2)
 
 
 @pytest.mark.parametrize("k,L,scoring,weighting,levelsup", [(10, 3, 0, 0, 1), (10, 3, 0, 0, 4), (6, 4, 1, 1, 2), (4, 5, 5, 0, 3), (7, 3, 2, 2, 0),
@@ -27,14 +26,14 @@ def test_transform_matches_the_reference_code(ref, k, L, scoring, weighting, lev
     with tempfile.TemporaryDirectory() as d:
         path = os.path.join(d, "voc.txt")
         ref.write_vocabulary_text(voc, path)
-        R = ref.RefVocabulary(path)
+        R = ref.obj("RefVocabulary", lambda: ref.RefVocabulary(path))
     O = ref.Vocabulary(voc)
     assert R.words() == int(np.asarray(voc["is_leaf"]).sum())
     a, b = O.transform(feat, levelsup), R.transform(feat, levelsup)
     for key in ("word", "weight", "bow_id", "bow_val", "fv_node_id", "fv_node_ptr", "fv_feat"):
-        assert np.array_equal(a[key], b[key]), key
+        assert same(a[key], b[key]), key
     if L - levelsup > 0:           # otherwise the reference leaves *nid untouched for non-root levels; both report the root
-        assert np.array_equal(a["node"], b["node"])
+        assert same(a["node"], b["node"])
     assert len(a["bow_id"]) > 20
     O.close(); R.close()
 

@@ -6,22 +6,22 @@ compared BIT FOR BIT: formulas, branch thresholds, expression grouping, float/do
 Compiling the reference this way found four places where the oracle's restatement differed in the last bits or in a threshold (each
 fixed in the oracle and noted there): RobustKernelHuber keeps delta^2 in a float; Sim3::log groups (B*Omega)*Omega; the point Jacobian
 groups ((-1/z)*tmp)*R; the pose-landmark block is B^T(A^T Omega)^T without a kernel and (B^T wOmega)A with one; the unary edge's b is
-((rho1 A^T) Omega) e.  Skipped where neither the reference tree nor a prebuilt library is present."""
+((rho1 A^T) Omega) e.  The reference's outputs are stored under tests/golden/reference (tests/reference_outputs.py)."""
 import numpy as np
 import pytest
 
 from ccm_slam_b200 import synth
+from tests.reference_outputs import Recorded, same
 
 
 @pytest.fixture(scope="module")
 def sides(oracle):
-    if oracle.ref_g2o() is None:
-        pytest.skip("reference tree absent and no prebuilt oracle/_ref/libg2o_types_ref.so")
-    return oracle.Pieces("oracle"), oracle.Pieces("ref"), oracle
+    rec = Recorded(oracle, __file__, oracle.ref_g2o)
+    return oracle.Pieces("oracle"), rec.obj("Pieces", lambda: oracle.Pieces("ref")), rec
 
 
 def eq(a, b):
-    return np.array_equal(np.asarray(a), np.asarray(b))
+    return same(a, b)
 
 
 def test_se3(sides):
@@ -46,7 +46,8 @@ def test_se3(sides):
         T[:3, :3] = Rotation.from_rotvec(rv).as_matrix().astype(np.float32); T[:3, 3] = np.float32([0.3, -1.2, 2.5])
         qt = orc.pose_from_Tcw_f32(T)
         assert eq(qt, R.vec("se3_from_Rt", 7, T[:3, :3].astype(np.float64).ravel(), T[:3, 3].astype(np.float64)))
-        assert eq(orc.pose_to_Tcw_f32(qt), R.vec("se3_homogeneous", 16, qt).astype(np.float32).reshape(4, 4))
+        to_f32 = lambda q: R.live.vec("se3_homogeneous", 16, q).astype(np.float32).reshape(4, 4)
+        assert eq(orc.pose_to_Tcw_f32(qt), orc.call("se3_homogeneous_f32", to_f32, qt))
 
 
 def test_sim3(sides):

@@ -2,11 +2,12 @@
 OptimizationAlgorithmLevenberg::solve (oracle/ref_lm_wrap.cpp: g2o's three optimization_algorithm*.cpp files compiled in place over
 stand-in SparseOptimizer / Solver classes whose bodies are the oracle's linear algebra).  Both drivers run the same arithmetic, so
 lambda, chi2, trial counts, iteration counts and the final state must agree to the last bit; anything else is a control-flow
-difference.  Skipped where neither the reference tree nor a prebuilt oracle/_ref/liblm_ref.so is present."""
+difference.  The reference's outputs are stored under tests/golden/reference (tests/reference_outputs.py)."""
 import numpy as np
 import pytest
 
 from ccm_slam_b200 import synth
+from tests.reference_outputs import Recorded, same
 
 
 class _Side:
@@ -26,9 +27,8 @@ class _Side:
 #          (oracle/ref_ba_block_wrap.cpp)
 @pytest.fixture(scope="module", params=["lm", "full", "block"])
 def ref(oracle, request):
-    if {"lm": oracle.ref_lm, "full": oracle.ref_ba_full, "block": oracle.ref_ba_block}[request.param]() is None:
-        pytest.skip("reference tree absent and no prebuilt oracle/_ref library")
-    return _Side(oracle, request.param)
+    live = {"lm": oracle.ref_lm, "full": oracle.ref_ba_full, "block": oracle.ref_ba_block}[request.param]
+    return _Side(Recorded(oracle, __file__, live, keep={"trace"}), request.param)
 
 
 def same_run(a, b):
@@ -37,10 +37,10 @@ def same_run(a, b):
     for c in (0, 1, 2, 4, 5):       # iteration, lambda of the last trial, robust chi2 kept, trials, lambda handed to the next iteration
         if c == 1 and np.isnan(b["trace"][:, 1]).all():
             continue                # with the reference's own BlockSolver the last trial's lambda is not visible from outside
-        assert np.array_equal(a["trace"][:, c], b["trace"][:, c]), c
+        assert same(a["trace"][:, c], b["trace"][:, c]), c
     assert a["chi2_initial"] == b["chi2_initial"] and a["chi2_final"] == b["chi2_final"] and a["lambda_final"] == b["lambda_final"]
-    assert np.array_equal(a["poses"], b["poses"]) and np.array_equal(a["points"], b["points"])
-    assert np.array_equal(a["chi2"], b["chi2"]) and np.array_equal(a["depth_pos"], b["depth_pos"])
+    assert same(a["poses"], b["poses"]) and same(a["points"], b["points"])
+    assert same(a["chi2"], b["chi2"]) and same(a["depth_pos"], b["depth_pos"])
 
 
 @pytest.mark.parametrize("name,iters,robust", [("tiny", 20, True), ("small", 20, True), ("small", 10, False), ("cfg2", 15, True)])

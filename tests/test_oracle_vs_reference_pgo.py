@@ -1,12 +1,14 @@
 """CPU suite: the oracle's essential-graph optimisation against a run where the REFERENCE'S OWN code does everything but the sparse
 factorisation: g2o's Levenberg-Marquardt driver over g2o's VertexSim3Expmap / EdgeSim3 — Sim3::log errors, the numeric Jacobians of
 BaseBinaryEdge::linearizeOplus, constructQuadraticForm into upper-triangle 7x7 blocks with the transposed write, oplus with _fix_scale
-(oracle/ref_pgo_full_wrap.cpp -> oracle/_ref/libpgo_full_ref.so).  Traces and final vertices bit for bit.  Skipped where neither the
-reference tree nor a prebuilt library is present."""
+(oracle/ref_pgo_full_wrap.cpp -> oracle/_ref/libpgo_full_ref.so).  Traces and final vertices bit for bit.  The reference's outputs are stored under
+tests/golden/reference (tests/reference_outputs.py)."""
 import numpy as np
 import pytest
 
 from ccm_slam_b200 import synth
+from tests.reference_outputs import Recorded
+from tests.reference_outputs import same as same_array
 
 
 class _Side:
@@ -19,9 +21,8 @@ class _Side:
 # the non-Schur solve) — only LinearSolver::solve, the sparse LDL^T, is the oracle's (oracle/ref_pgo_block_wrap.cpp)
 @pytest.fixture(scope="module", params=["full", "block"])
 def ref(oracle, request):
-    if (oracle.ref_pgo_full() if request.param == "full" else oracle.ref_pgo_block()) is None:
-        pytest.skip("reference tree absent and no prebuilt oracle/_ref library")
-    return _Side(oracle, request.param)
+    live = oracle.ref_pgo_full if request.param == "full" else oracle.ref_pgo_block
+    return _Side(Recorded(oracle, __file__, live, keep={"trace"}), request.param)
 
 
 def same(a, b):
@@ -29,9 +30,9 @@ def same(a, b):
     for c in (0, 1, 2, 4, 5):
         if c == 1 and np.isnan(b["trace"][:, 1]).all():
             continue                # inside the reference's own BlockSolver the last trial's lambda is not visible
-        assert np.array_equal(a["trace"][:, c], b["trace"][:, c]), c
+        assert same_array(a["trace"][:, c], b["trace"][:, c]), c
     assert a["chi2_initial"] == b["chi2_initial"] and a["chi2_final"] == b["chi2_final"] and a["lambda_final"] == b["lambda_final"]
-    assert np.array_equal(a["sim3"], b["sim3"])
+    assert same_array(a["sim3"], b["sim3"])
 
 
 @pytest.mark.parametrize("fix_scale", [False, True])
@@ -58,4 +59,4 @@ def test_fixed_vertices_stop_flag_and_empty(ref):
     same(ref.pgo_solve(p, iterations=0), ref.ref_pgo_solve(p, iterations=0))
     p.fixed[:] = 1
     a = ref.pgo_solve(p, iterations=5); b = ref.ref_pgo_solve(p, iterations=5)
-    assert a["iters_done"] == b["iters_done"] == -1 and np.array_equal(a["sim3"], b["sim3"])
+    assert a["iters_done"] == b["iters_done"] == -1 and same_array(a["sim3"], b["sim3"])

@@ -1,18 +1,18 @@
 """CPU suite: the oracle's PoseOptimizationClient and OptimizeSim3 against runs where the REFERENCE'S OWN code does everything but the
 6x6 / 7x7 Cholesky: g2o's Levenberg-Marquardt driver over g2o's VertexSE3Expmap / EdgeSE3ProjectXYZOnlyPose and VertexSim3Expmap /
 EdgeSim3ProjectXYZ / EdgeInverseSim3ProjectXYZ with Huber kernels (oracle/ref_single_full_wrap.cpp -> oracle/_ref/libsingle_full_ref.so).
-Estimates bit for bit, flags and counts exact.  Skipped where neither the reference tree nor a prebuilt library is present."""
+Estimates bit for bit, flags and counts exact.  The reference's outputs are stored under
+tests/golden/reference (tests/reference_outputs.py)."""
 import numpy as np
 import pytest
 
 from ccm_slam_b200 import synth
+from tests.reference_outputs import Recorded, same
 
 
 @pytest.fixture(scope="module")
 def ref(oracle):
-    if oracle.ref_single_full() is None:
-        pytest.skip("reference tree absent and no prebuilt oracle/_ref/libsingle_full_ref.so")
-    return oracle
+    return Recorded(oracle, __file__, oracle.ref_single_full)
 
 
 def pose_args(d):
@@ -28,9 +28,9 @@ def sim3_args(d, fix):
 def test_pose_optimization(ref, n, seed, frac, noise):
     d = synth.make_pose_opt(n=n, seed=seed, outlier_frac=frac, noise_px=noise)
     T, out, nin = ref.pose_optimize(*pose_args(d)); Tr, outr, ninr = ref.ref_pose_optimize(*pose_args(d))
-    assert nin == ninr and np.array_equal(out, outr) and np.array_equal(T, Tr)
+    assert nin == ninr and same(out, outr) and same(T, Tr)
     if n < 3:
-        assert nin == 0 and np.array_equal(T, d["Tcw0"])
+        assert nin == 0 and same(T, d["Tcw0"])
     if frac >= 0.15 and n >= 60:
         assert 0 < out.sum() < n
 
@@ -41,7 +41,7 @@ def test_pose_optimization_bad_start(ref):
     for seed in range(30, 36):
         d = synth.make_pose_opt(n=150, seed=seed, outlier_frac=0.25, pose_noise=(0.15, 0.5))
         a = ref.pose_optimize(*pose_args(d)); b = ref.ref_pose_optimize(*pose_args(d))
-        assert a[2] == b[2] and np.array_equal(a[1], b[1]) and np.array_equal(a[0], b[0])
+        assert a[2] == b[2] and same(a[1], b[1]) and same(a[0], b[0])
         hit += a[1].sum() > 40
     assert hit >= 1
 
@@ -51,8 +51,8 @@ def test_pose_optimization_bad_start(ref):
 def test_sim3_optimization(ref, n, seed, fix, frac):
     d = synth.make_sim3_opt(n=n, seed=seed, fix_scale=fix, outlier_frac=frac)
     S, inl, nin = ref.sim3_optimize(*sim3_args(d, fix)); Sr, inlr, ninr = ref.ref_sim3_optimize(*sim3_args(d, fix))
-    assert nin == ninr and np.array_equal(inl, inlr) and np.array_equal(S, Sr)
+    assert nin == ninr and same(inl, inlr) and same(S, Sr)
     if n < 10:
-        assert nin == 0 and np.array_equal(S, d["S12_0"])        # fewer than 10 pairs survive: g2oS12 is left alone
+        assert nin == 0 and same(S, d["S12_0"])        # fewer than 10 pairs survive: g2oS12 is left alone
     if fix and nin:
         assert S[7] == d["S12_0"][7]
